@@ -3,7 +3,7 @@
 120 000-triangle random-cube scene (create_n_cubes(10 000), src/testbase.rs:608-615), 1 M create_ray rays
 (src/testbase.rs:687-691), f32/3D.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--no-extras]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--no-extras] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path's query side over one ray batch: batched Bvh::traverse of 1 M rays
 against the device-resident tree, producing the CSR hit lists.  At N > 1 every rank traverses its own
@@ -309,6 +309,15 @@ def run_b200(args):
     sampler.mark_end()
     launches = ctx.launch_count() - launches0
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:      # the CSR of the last timed step, before anything else writes the buffers
+        if sharded is None:
+            off = d_off.cpu().numpy().view(np.uint32)
+            if int(off[-1]) > cap:
+                raise SystemExit(f"--dump-outputs: {int(off[-1])} hits do not fit the hit buffer (cap {cap})")
+            hits = d_hits[: int(off[-1])].cpu().numpy().view(np.uint32)
+        else:
+            off, hits = sharded.fetch()
+        _dump_outputs(args.dump_outputs, np, off, hits)
     mine = [a.elapsed_time(b) for a, b in ev]
     job_ms, rank_medians = per_step_max(mine)
     spread = _stats(job_ms)
@@ -428,6 +437,24 @@ def run_b200(args):
                             "sample": f"{leg['sample']} rays x {leg['steps']} back-to-back reps, sustained rate (total rays / wall time), Bvh::traverse (recursive), persistent pinned pool of {leg['threads']} threads, dynamic chunks",
                             "build_Mprims_per_s_1thread": leg["build_1"], "build_Mprims_per_s_all_threads": leg["build_all"]}
     print(json.dumps(line), flush=True)
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def _dump_outputs(out_dir: str, np, offsets, hits):
+    """Writes the CSR a caller of the traversal receives as out_dir/offsets.npy and out_dir/hits.npy, both float32: every offset
+    is at most the hit-buffer capacity (<= 16 M < 2**24) and every hit is a shape index (120 000 shapes), so the values are exact."""
+    arrays = {"offsets": offsets, "hits": hits}
+    for name, a in arrays.items():
+        if len(a) and int(a.max()) >= 1 << 24:
+            raise SystemExit(f"--dump-outputs: {name} holds values float32 cannot represent exactly")
+    nbytes = sum(4 * len(a) for a in arrays.values())
+    if nbytes > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"--dump-outputs: {nbytes} bytes exceed the {DUMP_LIMIT_BYTES}-byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float32))
 
 
 def _sharded_parity(torch, dist, np, bvh, sharded, d_rays, d_off, d_hits, cap, rank, world, dev) -> bool:
@@ -727,7 +754,11 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-extras", action="store_true", help="skip the sponza16M / hbm_bound extras")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the CSR hit lists of the last timed step (global CSR at N > 1) as DIR/offsets.npy and "
+                                                          "DIR/hits.npy (float32); the inputs are seeded, so two builds can be compared output for output")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -47,9 +47,13 @@ def test_no_cpu_fallback_without_a_device():
 
 
 def test_library_contains_only_sm100a_code():
-    from bvh_b200 import capi
+    import shutil
 
-    out = subprocess.run(["cuobjdump", "--list-elf", capi.SO_PATH], capture_output=True, text=True).stdout
+    from bvh_b200 import build, capi
+
+    # the toolkit that built the library, which need not be on PATH
+    cuobjdump = shutil.which("cuobjdump", path=os.path.dirname(build.NVCC) or None) or "cuobjdump"
+    out = subprocess.run([cuobjdump, "--list-elf", capi.SO_PATH], capture_output=True, text=True).stdout
     archs = set(l.split(".")[-2] for l in out.splitlines() if ".cubin" in l)
     assert archs == {"sm_100a"}, archs
 
